@@ -20,6 +20,9 @@ random-init weights of the named architecture (no checkpoints are reachable offl
   --config s2tt    : BASELINE configs[1] (8 x 10 s, encoder + text decoder only).
   --config stream  : BASELINE configs[4] (SeamlessStreaming EMMA S2ST, one 30 s synthetic stream in 320 ms segments): compute
                      latency per source segment and the real-time factor.
+  --dump-outputs DIR : after the timed steps, writes what the last timed step returned to its caller as DIR/<name>.npy
+                     (dump_outputs).  Inputs and weights are seeded, so two builds run with the same arguments can be
+                     compared output for output.
 """
 import argparse
 import ctypes
@@ -52,6 +55,48 @@ STREAM_WORKLOAD = ("SeamlessStreaming S2ST (EMMA monotonic text decoder dense_1b
 # algorithmic work per 10 s utterance at L=102, U=495 (SURVEY 8d / BASELINE.md 2)
 GFLOP_PER_UTT = {"encoder": 618.9, "t2u": 155.0, "vocoder": 165.0}
 FBANK_BYTES_PER_UTT = 0.80e6
+DUMP_BYTES = 60 << 20  # array data written by --dump-outputs, all files together
+
+
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"{s} is not >= 1")
+    return v
+
+
+def dump_outputs(out_dir, texts=None, text_ids=None, units=None, wavs=None):
+    """Writes one step's outputs as out_dir/<name>.npy: texts as Unicode code points and token / unit ids as float64
+    (exact), waveforms as float32.  Each is a list of 1-D rows, stored padded to a rectangle (-1 for ids, 0 for audio)
+    with the row lengths in <name>_lengths.npy.  If the waveforms would take the data past DUMP_BYTES, a fixed seeded
+    sample of their time positions is kept, listed in audio_wavs_positions.npy."""
+    import numpy as np
+
+    def rect(rows, pad, dtype):
+        lens = np.array([len(r) for r in rows], dtype=np.float64)
+        a = np.full((len(rows), int(lens.max(initial=0))), pad, dtype=dtype)
+        for i, r in enumerate(rows):
+            a[i, :len(r)] = r
+        return a, lens
+
+    arrays = {}
+    if texts is not None:
+        arrays["texts"], arrays["texts_lengths"] = rect([[ord(c) for c in t] for t in texts], -1, np.float64)
+    if text_ids is not None:
+        arrays["text_ids"], arrays["text_ids_lengths"] = rect(text_ids, -1, np.float64)
+    if units is not None:
+        arrays["units"], arrays["units_lengths"] = rect(units, -1, np.float64)
+    if wavs is not None:
+        w, lens = rect([x.detach().flatten().float().cpu().numpy() for x in wavs], 0, np.float32)
+        room = DUMP_BYTES - sum(a.nbytes for a in arrays.values()) - lens.nbytes
+        if w.nbytes > room:
+            keep = room // (4 * w.shape[0] + 8)
+            pos = np.sort(np.random.default_rng(0).choice(w.shape[1], size=keep, replace=False))
+            w, arrays["audio_wavs_positions"] = w[:, pos], pos.astype(np.float64)
+        arrays["audio_wavs"], arrays["audio_wavs_lengths"] = w, lens
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def peaks():
@@ -223,7 +268,9 @@ def run_reference(args, rank):
     if rank != 0:
         return
     cfg = CONFIGS[args.config]
-    block, _ = cpu_baseline_block(cfg["task"], 4, max(1, min(args.steps, 3)), warmup=args.warmup > 0)
+    block, out = cpu_baseline_block(cfg["task"], 4, args.steps, warmup=args.warmup > 0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, texts=out["texts"], units=out.get("speech_units"), wavs=out.get("wavs"))
     v = block["value"]
     line = {"impl": "reference", "metric": cfg["metric"], "value": v, "unit": "utt/s", "n_gpus": args.gpus,
             "steps": len(block["seconds_per_run"]), "warmup": 1 if args.warmup > 0 else 0,
@@ -231,7 +278,7 @@ def run_reference(args, rank):
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": workload_config(cfg, cfg["batch"], max(1, args.gpus)),
             "sample": "each step = batch 4 of the workload's utterances on the host CPU (BASELINE.md 3 protocol: 1 warm-up, "
-                      "at most 3 timed runs, thread count = fastest of a probe)",
+                      "--steps timed runs, thread count = fastest of a probe)",
             "cpu_baseline": block,
             "e2e": {"value": v, "unit": "utt/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     print(json.dumps(line))
@@ -400,12 +447,14 @@ def run_stream(args, device):
     mono = load_monotonic_decoder_model("base_v2", device=device, state_dict=S.make_monotonic_state_dict(cfg, seed=2), tokenizers=toks)
     wave = torch.cat([w for w in S.make_waveforms(3, SAMPLES, seed=4321)])  # 30 s
     results = []
-    for rep in range(max(1, args.warmup) + max(1, min(args.steps, 3))):
+    for rep in range(max(1, args.warmup) + args.steps):
         st = StreamingS2ST(tr.model, mono, tr.vocoder, TGT_LANG)
         torch.cuda.synchronize()
         ids, chunks = st.run(wave)
         results.append(st)
     timed = results[max(1, args.warmup):]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, text_ids=[ids], wavs=[torch.cat([c.flatten() for c in chunks]) if chunks else torch.zeros(0)])
     lat = sorted(x for st in timed for x in st.latencies_ms)
     total_ms = statistics.mean(sum(st.latencies_ms) for st in timed)
     st = timed[-1]
@@ -427,8 +476,9 @@ def run_stream(args, device):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=12)
+    ap.add_argument("--steps", type=positive_int, default=12, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--config", default="s2st", choices=sorted(CONFIGS) + ["stream"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -498,15 +548,17 @@ def main():
     main_stream = torch.cuda.current_stream()
 
     def run_device_steps(n):
-        """n steps, each one batch through the whole path; with lanes, LANES of them are in flight at any time."""
+        """n steps, each one batch through the whole path; with lanes, LANES of them are in flight at any time.
+        Returns what the last step returned."""
         if pool is None:
             for _ in range(n):
-                step_device()
-            return
+                out = step_device()
+            return out
         futs = [pool.submit(i, step_device) for i in range(n)]
         for f in futs:
-            _, done = f.result()
+            out, done = f.result()
             main_stream.wait_event(done)
+        return out
 
     # ---- device-resident leg
     if pool is not None:
@@ -518,13 +570,17 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     torch.cuda.synchronize()
     e0.record()
-    run_device_steps(args.steps)
+    last = run_device_steps(args.steps)
     e1.record()
     sync_all()
     ms_dev = max_over_ranks(e0.elapsed_time(e1) / args.steps)
     launches_total = launches_now() - n0  # kernels of this library launched inside the timed region (graph replays included)
     launches = launches_total // args.steps
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        texts, speech = last
+        dump_outputs(args.dump_outputs, texts=texts, units=speech.units if speech is not None else None,
+                     wavs=speech.audio_wavs if speech is not None else None)
 
     # one batch at a time (no lanes): the latency of a step and the reference point for the lanes' gain
     step_device()

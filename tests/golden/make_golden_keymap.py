@@ -16,6 +16,7 @@ its groups instantiated), plus the entries the function deletes / rewrites.  The
 for the rewritten tensors, checksums - regenerated deterministically by the test from the same seeds."""
 import ast
 import json
+import math
 import os
 import re
 import sys
@@ -90,8 +91,10 @@ def make_inputs(key_map):
 
 
 def checksum(t):
-    t = t.double()
-    return [list(t.shape), float(t.sum()), float((t * torch.arange(1, t.numel() + 1, dtype=torch.float64).view(t.shape)).sum())]
+    """Shape, sum and position-weighted sum.  The products are exact in float64 and math.fsum rounds the exact sum, so
+    the value does not depend on the order in which a host's torch.sum happens to reduce."""
+    v = t.double().flatten()
+    return [list(t.shape), math.fsum(v.tolist()), math.fsum((v * torch.arange(1, v.numel() + 1, dtype=torch.float64)).tolist())]
 
 
 def main():

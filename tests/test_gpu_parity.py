@@ -859,14 +859,23 @@ def test_full_width_s2st_matches_oracle(base, ops):
         if s + 1 < len(trace["inputs"]):
             assert toks == trace["inputs"][s + 1].tolist(), f"step {s}: tokens differ"
     assert [f[1] for f in finished] == [f[1] for f in trace["finished"]]
-    # --- a11-a14: units from the oracle's decoder states (upstream near ties cannot mask a defect)
-    dseq = Seq(1, ref["dec_out"].shape[1], M, lens=tl, buf=ref["dec_out"].to(dev).half().reshape(-1, M).contiguous())
+    # --- a11-a14: units from the oracle's decoder states (upstream near ties cannot mask a defect).  The fp16 states come
+    # from a fixture of this same oracle run (tests/golden/make_golden_full_width.py): recomputed here they move by ~1e-4
+    # with the host's threads and ISA, which changes their fp16 rounding and with it units at near ties
+    g = np.load(os.path.join(G, "full_width_t2u_ref.npz"))
+    g_dec, g_units = torch.from_numpy(g["dec_out"]), torch.from_numpy(g["units"])
+    assert rel(ref["dec_out"], g_dec) < 1e-3, "the oracle's decoder states no longer match the fixture"  # fp16 rounding
+    for k in ("text_seqs", "dur", "unit_lens", "units"):
+        assert torch.equal(ref[k], torch.from_numpy(g[k])), f"the oracle's {k} no longer match the fixture"
+    dseq = Seq(1, g_dec.shape[1], M, lens=tl, buf=g_dec.to(dev).reshape(-1, M).contiguous())
     units, ulens, _ = eng.t2u(dseq, ref["text_seqs"].to(dev), durations=ref["dur"])
     assert ulens.tolist() == ref["unit_lens"].tolist()
     n = int(ref["unit_lens"][0])
     assert n == 495  # 99 subwords x 5 characters, duration 1 each (SURVEY 8d)
-    diff = int((units[0, :n].cpu() != ref["units"][0, :n]).sum())
-    assert diff <= 1, f"{diff} unit ids differ from the oracle"
+    differ = (units[0, :n].cpu() != g_units[0, :n]).nonzero().flatten().tolist()
+    diff = len(differ)
+    assert diff <= 1, (f"{diff} unit ids differ from the oracle at {differ} "
+                       f"(oracle top-2 margins {[round(float(g['unit_margins'][i]), 5) for i in differ]})")
     # --- a15/a16: waveform from the oracle's units, and the trimming rule
     wav = voc(ref["units"].to(dev), "spa", -1, dur_prediction=False)
     err_wav = (wav.float().cpu() - ref["wav_full"]).abs().max().item()
